@@ -5,7 +5,7 @@ A *step* is one raft tick over every group of the job: the fused sm_100a tick ke
 append-acks / votes, applies proposals, runs the matchIndex -> commitIndex quorum (q-th largest of the
 replica columns, term-gated) and the election timers, for all groups at once (SURVEY §8a rows a3-a16).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 N > 1 is launched by the driver under torch.distributed.run (one rank per GPU); the groups are sharded
 contiguously (strong scaling: the job stays 1,048,576 groups) and every tick ends with one all-gather of
@@ -368,9 +368,24 @@ def run_ours(args):
     def eng_mode():
         return cur_mode[0]
 
-    def timed_leg(tick_mode, graph, write_through=1, nreps=reps, sample_clocks=False):
+    def last_step_outputs(tick_mode):
+        """What a caller of the timed path reads after its last tick: every group's commit index, that tick's out words
+        (and in tick mode 4 its commit advances), and the term / role / last index columns.  float64 holds the u64 indices
+        exactly (they stay below 2^53); 40 B per group, 40 MB at 1,048,576 groups."""
+        st = eng.export_state(("term", "role", "last_index"))
+        got = {"committed": eng.sync_commits().astype(np.float64), "out": eng.sync_out().astype(np.float64),
+               "term": st["term"].astype(np.float64), "role": st["role"].astype(np.float32),
+               "last_index": st["last_index"].astype(np.float64)}
+        if tick_mode == 4:
+            got["commit_advance"] = eng.sync_tick_deltas().astype(np.float32)
+        return got
+
+    dumped = {}
+
+    def timed_leg(tick_mode, graph, write_through=1, nreps=reps, sample_clocks=False, dump=False):
         """`nreps` repetitions of: rewind, W warm-up ticks, then EXACTLY K ticks between barrier + synchronize, CUDA
-        events on the engine's stream, max over ranks.  Returns (median ms for K ticks, all reps, launches, clocks)."""
+        events on the engine's stream, max over ranks.  Returns (median ms for K ticks, all reps, launches, clocks).
+        With `dump`, the outputs of the last rep's last tick go to `dumped` (every rep replays the same inputs)."""
         out_ms, launches, clocks = [], 0, None
         cur_mode[0] = tick_mode
         rewind(tick_mode, graph, write_through)  # rehearsal (untimed): graphs captured, descriptor tables built
@@ -398,6 +413,8 @@ def run_ours(args):
                 dist.all_reduce(t, op=dist.ReduceOp.MAX)
                 ms = float(t.item())
             out_ms.append(ms)
+        if dump:
+            dumped.update(last_step_outputs(tick_mode))
         med = float(np.median(out_ms))
         if sampler is not None:
             # keep the GPU under the tick kernels ~2 s more so that the sampler sees it at the clocks of the timed region
@@ -443,7 +460,8 @@ def run_ours(args):
             n_escapes += len(wide8)
             eng.post_inbox_packed(w8, p8, wide8, slot=t, keep=True)
 
-    ms, ms_reps, launches_timed, clocks = timed_leg(mode, graph, wt, sample_clocks=True)
+    dump_dir = getattr(args, "dump_outputs", None) if rank == 0 else None  # N > 1: rank 0's shard
+    ms, ms_reps, launches_timed, clocks = timed_leg(mode, graph, wt, sample_clocks=True, dump=bool(dump_dir))
     ticks_per_s = K / (ms / 1e3)
     peak, peak_src = measured_peak_gbs()
     batched = mode == 4 and graph != 0 and not (world > 1 and args.gather == "nccl")  # (a per-tick ncclAllGather forces per-tick launches)
@@ -546,6 +564,10 @@ def run_ours(args):
         if rank == 0:
             line["e2e"] = e2e
     eng.close()
+    if dump_dir:
+        os.makedirs(dump_dir, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(dump_dir, f"{name}.npy"), a)
     if rank == 0:
         print(json.dumps(line))
     if dist is not None:
@@ -800,7 +822,13 @@ def main():
     ap.add_argument("--weak", action="store_true",
                     help="N>1: weak scaling — every GPU keeps 1,048,576 groups, the job is N times that (default: the job "
                          "stays 1,048,576 groups, BASELINE configs[3]); compare group_ticks_per_sec across N")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--impl ours: after the timed ticks, write what the last one computed as DIR/<name>.npy (float32 / "
+                         "float64): commit indices, out words, commit advances, term, role, last index; the inputs are "
+                         "seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

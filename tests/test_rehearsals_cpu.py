@@ -162,6 +162,33 @@ def test_rehearse_bench_inbox_forms_replay_the_same_ticks(monkeypatch, capsys):
     assert (finals["wide"] > bench.steady_state(2048, bench.R, 0, bench.SEED)["committed"]).mean() > 0.9
 
 
+def test_rehearse_bench_dump_outputs(monkeypatch, capsys, tmp_path):
+    """`bench.py --dump-outputs DIR` writes what the last timed tick computed, as float32 / float64 .npy files"""
+    import numpy as np
+
+    from engine_double import FakeBenchEngine
+
+    at_stop = []
+
+    class Eng(FakeBenchEngine):
+        def timer_stop(self):  # the end of a timed region
+            at_stop.append(self.o.export())
+            return super().timer_stop()
+
+    monkeypatch.setenv("MRQ_BENCH_FAST", "1")  # the headline leg alone: its last rep is the last timed region
+    bench, made = _bench_on_the_double(monkeypatch, Eng)
+    bench.run_ours(_args(dump_outputs=str(tmp_path / "dump")))
+    capsys.readouterr()
+    got = {p.stem: np.load(p) for p in (tmp_path / "dump").glob("*.npy")}
+    assert set(got) == {"committed", "out", "term", "role", "last_index", "commit_advance"}
+    assert all(a.dtype in (np.float32, np.float64) and a.shape == (2048,) for a in got.values())
+    want = at_stop[-1]
+    for k in ("committed", "out", "term", "role", "last_index"):
+        np.testing.assert_array_equal(got[k], want[k], err_msg=k)
+    assert (got["committed"] > bench.steady_state(2048, bench.R, 0, bench.SEED)["committed"]).mean() > 0.9
+    assert got["commit_advance"].max() > 0
+
+
 @pytest.mark.parametrize("G,R,cfg", [(1200, 7, 5), (900, 5, 3), (300, 2, 5), (64, 1, 2)])
 def test_rehearse_gpu_test_mode_4_per_tick(monkeypatch, G, R, cfg):
     import test_zz_compact_gpu as t
